@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — 1080p frames/sec of the Motion (Laplace, 6-level) hot path on N B200s.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
   (N>1: launched by torchrun, one rank per GPU, NCCL; weak scaling — every rank serves its own
    `lanes` independent streams; the only collective on the data path is a one-time broadcast of the
    parameter block.)
@@ -12,6 +12,11 @@ through the public host API (pinned host frames in, pinned host frames out, copi
 timed region).  `--impl reference` times the reference's own CPU implementation of the path (its sources
 compiled in place into oracle/_ref, OpenCV kernels through cv2, all host threads; the oracle restatement if that
 module is absent) on the same workload.
+
+`--dump-outputs DIR` writes, after the timed steps, a fixed seeded sample of the frames the last device-resident step
+produced (DIR/output.npy, float32) with their flat indices into the [lanes, H, W, 3] output (DIR/output_index.npy,
+float64) and that shape (DIR/output_shape.npy).  The clip is synthetic and the sample's seed fixed, so two builds run
+with the same arguments can be compared value for value.
 """
 import argparse
 import ctypes as C
@@ -120,6 +125,24 @@ def make_clip(t_frames, lanes):
         for k in range(lanes):
             clip[t, k] = np.roll(base[t], (11 * k, 37 * k), axis=(0, 1))
     return clip
+
+
+DUMP_SAMPLES, DUMP_SEED = 1 << 22, 20240611   # <= 48 MB of float32 values + float64 indices
+
+
+def dump_outputs(out_d, out_dir):
+    """Writes a seeded sample of the device output tensor out_d (uint8, any shape) to out_dir as float32 / float64 .npy."""
+    import torch
+    total = out_d.numel()
+    if total <= DUMP_SAMPLES:
+        idx = np.arange(total, dtype=np.int64)
+    else:
+        idx = np.sort(np.random.default_rng(DUMP_SEED).choice(total, DUMP_SAMPLES, replace=False, shuffle=False))
+    vals = out_d.reshape(-1)[torch.from_numpy(idx).to(out_d.device)].cpu().numpy()
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "output.npy"), vals.astype(np.float32))
+    np.save(os.path.join(out_dir, "output_index.npy"), idx.astype(np.float64))
+    np.save(os.path.join(out_dir, "output_shape.npy"), np.array(out_d.shape, np.float64))
 
 
 def oracle_cfg():
@@ -379,6 +402,8 @@ def run_ours(args, rank, world, local_rank):
     barrier()
     sampler.window(t_w0, time.time())
     ms = max_over_ranks(e0.elapsed_time(e1))
+    if args.dump_outputs and rank == 0:      # out_d holds the last timed step's frames
+        dump_outputs(out_d, args.dump_outputs)
     from lvm_b200.shard import sum_over_ranks
     launches = int(sum_over_ranks(float(proc.launch_count - l0), dist, device="cuda"))
     fps = world * lanes * args.steps / (ms * 1e-3)
@@ -544,7 +569,11 @@ def main():
     ap.add_argument("--opt", action="append", default=[], help="library option key=value (mc_set_option), repeatable")
     ap.add_argument("--workload", default="1080p6", choices=["1080p6", "4k8"],
                     help="1080p6 = BASELINE.json configs[1] (the headline, default); 4k8 = configs[4]: 3840x2160, 8 levels")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write a seeded sample of the last timed step's output frames to DIR as .npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     if args.workload == "4k8":       # BASELINE.json configs[4]: a parity-test case, reported as an extra line on request
         global W, H, LEVELS, WORKLOAD
         W, H, LEVELS = 3840, 2160, 8

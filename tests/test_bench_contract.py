@@ -65,10 +65,10 @@ def test_kernel_table_accounting():
 
 
 @pytest.mark.emu
-def test_product_arm_dry_run_on_emulation(monkeypatch):
-    """bench.run_ours end to end (device-resident loop, pipelined e2e loop, per-kernel table, CPU baseline, JSON line)
-    with the kernels on the CUDA-on-CPU emulation and a stand-in for the handful of torch.cuda calls it makes, at a
-    tiny frame size.  Guards the bench's own logic in the GPU-less container; the numbers mean nothing."""
+def test_product_arm_dry_run_on_emulation(monkeypatch, tmp_path):
+    """bench.run_ours end to end (device-resident loop, output dump, pipelined e2e loop, per-kernel table, CPU baseline,
+    JSON line) with the kernels on the CUDA-on-CPU emulation and a stand-in for the handful of torch.cuda calls it
+    makes, at a tiny frame size.  Guards the bench's own logic in the GPU-less container; the numbers mean nothing."""
     import time
     import types
     if torch.cuda.is_available():
@@ -105,7 +105,7 @@ def test_product_arm_dry_run_on_emulation(monkeypatch):
     monkeypatch.setitem(bench.UI, "levels", 4)
     try:
         args = types.SimpleNamespace(gpus=1, steps=3, warmup=3, lanes=2, clip_frames=2, cpu_frames=2, no_cpu_baseline=False,
-                                     ref_frames_per_step=1, opt=[], workload="1080p6")
+                                     ref_frames_per_step=1, opt=[], workload="1080p6", dump_outputs=str(tmp_path / "out"))
         d = json.loads(bench.run_ours(args, 0, 1, 0))
     finally:
         capi.LIB_PATH, capi._lib = saved
@@ -117,3 +117,26 @@ def test_product_arm_dry_run_on_emulation(monkeypatch):
     assert r["bound"] == "hbm" and 0 < r["frac"] and r["fused_level_kernel"]["kernel"] == "level[1]"
     assert {k["kernel"] for k in r["kernels"]} >= {"ingest_lab[0]", "egress[0]", "level[1]", "level[2]", "level[3]", "collapse[2]"}
     assert d["cpu_baseline"]["value"] > 0 and d["cpu_baseline"]["kind"] in ("reference", "port")
+    # 2 lanes of 192x108x3 fit the sample: the whole last output, in order
+    import numpy as np
+    vals, idx = np.load(tmp_path / "out" / "output.npy"), np.load(tmp_path / "out" / "output_index.npy")
+    assert vals.dtype == np.float32 and idx.dtype == np.float64
+    assert np.load(tmp_path / "out" / "output_shape.npy").tolist() == [2, 108, 192, 3]
+    assert np.array_equal(idx, np.arange(2 * 108 * 192 * 3)) and 0 <= vals.min() and vals.max() <= 255 and vals.std() > 0
+
+
+def test_dump_outputs_sample_is_fixed():
+    """bench.dump_outputs: above its sample size the same seeded positions are written every time, within 64 MB."""
+    import tempfile
+    import numpy as np
+    sys.path.insert(0, ROOT)
+    import bench
+    out = torch.from_numpy(np.random.default_rng(1).integers(0, 256, (3, 1080, 1920, 3), dtype=np.uint8))
+    with tempfile.TemporaryDirectory() as a, tempfile.TemporaryDirectory() as b:
+        bench.dump_outputs(out, a)
+        bench.dump_outputs(out, b)
+        idx = np.load(os.path.join(a, "output_index.npy"))
+        assert np.array_equal(idx, np.load(os.path.join(b, "output_index.npy")))
+        assert len(idx) == bench.DUMP_SAMPLES and np.all(np.diff(idx) > 0)
+        assert np.array_equal(np.load(os.path.join(a, "output.npy")), out.numpy().reshape(-1)[idx.astype(np.int64)])
+        assert sum(os.path.getsize(os.path.join(a, f)) for f in os.listdir(a)) <= 64 << 20

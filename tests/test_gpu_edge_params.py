@@ -1,8 +1,8 @@
-"""Parameter and size corner cases through all three modes, checked against the reference's own compiled code
-(oracle/_ref/_livim_ref; the oracle restatement if that module is absent): single-level pyramids, clamped level
-counts, zero amplification, thresholds at 0 and pi, cutoffs at 0 Hz / Nyquist / beyond (degenerate Butterworth design),
-inverted cutoffs, a 1 fps window, black frames (Color: 0/0 in the min-max stretch), 7x9 frames.  Passthrough decisions
-must be identical; outputs <= 1 LSB (Phase: <= 3 LSB, >= 99.5 % identical)."""
+"""Parameter and size corner cases through all three modes, checked against what the original project's own code
+returned (reproduced by the oracle, held bit-exact to the original through stored digests, tests/refpin.py):
+single-level pyramids, clamped level counts, zero amplification, thresholds at 0 and pi, cutoffs at 0 Hz / Nyquist /
+beyond (degenerate Butterworth design), inverted cutoffs, a 1 fps window, black frames (Color: 0/0 in the min-max
+stretch), 7x9 frames.  Passthrough decisions must be identical; outputs <= 1 LSB (Phase: <= 3 LSB, >= 99.5 % identical)."""
 import numpy as np
 import pytest
 
@@ -11,9 +11,9 @@ from lvm_b200.synth import synth_frame
 from oracle import livim_oracle as O
 from oracle import livim_ref
 from common import make_cfgs, u8_diff
+from refpin import ref_pin  # noqa: F401  (fixture)
 
 pytestmark = pytest.mark.gpu
-R = livim_ref.load()
 
 
 def clip(w, h, n, fps=30.0):
@@ -47,7 +47,7 @@ CASES = [
 
 
 @pytest.mark.parametrize("name,mode,ui,fps,special", CASES, ids=[c[0] for c in CASES])
-def test_corner_case_matches_reference(name, mode, ui, fps, special):
+def test_corner_case_matches_reference(name, mode, ui, fps, special, ref_pin):
     cfg, ocfg = make_cfgs(mode, *ui, fps)
     if special == "black":
         frames = [np.zeros((64, 96, 3), np.uint8) for _ in range(4)]
@@ -55,14 +55,11 @@ def test_corner_case_matches_reference(name, mode, ui, fps, special):
         frames = clip(7, 9, 3, fps)
     else:
         frames = clip(96, 64, 6 if mode == O.MODE_COLOR else 4, fps)
-    proc = L.MagnificationProcessor(0)
-    if R is not None:
-        ref, rcfg = R.Processor(), livim_ref.to_ref_config(R, ocfg)
-    else:
-        ref, rcfg = O.MagnificationProcessor(), ocfg
+    proc, ref, oproc = L.MagnificationProcessor(0), ref_pin.ref(lambda R: R.Processor()), O.MagnificationProcessor()
+    rcfg = livim_ref.to_ref_config(ref_pin.R, ocfg) if ref_pin.R is not None else None
     for t, f in enumerate(frames):
+        rprod, rout = ref_pin.process(ref, oproc, f, ocfg, rcfg, t)
         produced, out = proc.process_image(f, cfg)
-        rprod, rout = ref.process(f, rcfg)
         assert produced == bool(rprod), (name, t)
         if produced:
             d = u8_diff(out, rout)
