@@ -593,9 +593,9 @@ __device__ __forceinline__ float band_at(const BandSrc& b, size_t off) {
     return b.b ? band_of(v, __ldg(b.b + off), b.gain) : v;
 }
 
-__global__ void __launch_bounds__(256) k_collapse(Level lf, Level lc, BandSrc fine, BandSrc coarse, float* out) {
+__global__ void __launch_bounds__(256) k_collapse(Level lf, Level lc, BandSrc fine, BandSrc coarse, float* out, int plane_step) {
     __shared__ __align__(16) float sD[DH][DP];
-    const int plane = blockIdx.z;
+    const int plane = blockIdx.z * plane_step;
     const int x0 = blockIdx.x * TW, y0 = blockIdx.y * TH;
     const size_t cbase = (size_t)plane * lc.plane;
     for (int i = threadIdx.x; i < DH * DW; i += 256) {
@@ -694,13 +694,13 @@ __device__ __forceinline__ EgressIn<1> egress_load<1>(const EgressArgs& a, int l
 
 // `up` holds the pyrUp tap sums BEFORE their 1/64 scale: the scale is exact, so it is folded into the add (L) and
 // into the chroma factor (a, b) without changing a bit.  q / f: the row's output pointers at column gx (f may be null).
-template <int C>
-__device__ __forceinline__ void egress_convert(const EgressArgs& a, uint8_t* q, float* f, int gx, const EgressIn<C>& in, const float (&up)[C][4]);
-template <>
-__device__ __forceinline__ void egress_convert<3>(const EgressArgs& a, uint8_t* q, float* f, int gx, const EgressIn<3>& in, const float (&up)[3][4]) {
+// MC: channels of the motion image — 3, or 1 (L only) when chroma is 0: the attenuated a and b motion is then +-0 and
+// input + motion is the input itself, bit for bit (DESIGN §4), so A and B pass through.
+template <int MC>
+__device__ __forceinline__ void egress_convert(const EgressArgs& a, uint8_t* q, float* f, int gx, const EgressIn<3>& in, const float (&up)[MC][4]) {
+    static_assert(MC == 1 || MC == 3, "motion channels");
     uint8_t o8[12];
     float of[12];
-    const float chroma64 = a.chroma * kInv64;
     const short vL[4] = {in.L.x, in.L.y, in.L.z, in.L.w}, vA[4] = {in.A.x, in.A.y, in.A.z, in.A.w}, vB[4] = {in.B.x, in.B.y, in.B.z, in.B.w};
 #pragma unroll
     for (int i = 0; i < 4; ++i) {
@@ -710,11 +710,14 @@ __device__ __forceinline__ void egress_convert<3>(const EgressArgs& a, uint8_t* 
         if (a.m1.a) {
             // a,b motion planes *= chromAttenuation, then output = input + motion (MagnifyCore.hpp:140-148)
             L = __fmaf_rn(up[0][i], kInv64, L);
-            A = __fadd_rn(A, __fmul_rn(up[1][i], chroma64));   // the reference scales the plane, then adds
-            B = __fadd_rn(B, __fmul_rn(up[2][i], chroma64));
+            if constexpr (MC == 3) {
+                const float chroma64 = a.chroma * kInv64;
+                A = __fadd_rn(A, __fmul_rn(up[1][i], chroma64));   // the reference scales the plane, then adds
+                B = __fadd_rn(B, __fmul_rn(up[2][i], chroma64));
+            }
         }
         float ob, og, orr;
-        lab_to_bgr_fast(L, A, B, a.coeffs, a.gtab, ob, og, orr);
+        lab_to_bgr_fast<false, true>(L, A, B, a.coeffs, a.gtab, ob, og, orr);
         of[3 * i] = ob; of[3 * i + 1] = og; of[3 * i + 2] = orr;
         // lab_to_bgr clips to [0,1] before the gamma spline, so the saturating branches of
         // convertTo reduce to a min with 255 (NaN -> 0 by the conversion itself)
@@ -736,8 +739,7 @@ __device__ __forceinline__ void egress_convert<3>(const EgressArgs& a, uint8_t* 
             if (gx + i / 3 < a.w0) f[i] = of[i];
     }
 }
-template <>
-__device__ __forceinline__ void egress_convert<1>(const EgressArgs& a, uint8_t* q, float* f, int gx, const EgressIn<1>& in, const float (&up)[1][4]) {
+__device__ __forceinline__ void egress_convert(const EgressArgs& a, uint8_t* q, float* f, int gx, const EgressIn<1>& in, const float (&up)[1][4]) {
     uint8_t o8[4];
     float of[4];
 #pragma unroll
@@ -761,19 +763,20 @@ __device__ __forceinline__ void egress_convert<1>(const EgressArgs& a, uint8_t* 
     }
 }
 
-template <int C>
-__device__ __forceinline__ void egress_pixels(const EgressArgs& a, int lane, int gy, int gx, const float (&up)[C][4]) {
+template <int C, int MC>
+__device__ __forceinline__ void egress_pixels(const EgressArgs& a, int lane, int gy, int gx, const float (&up)[MC][4]) {
     const EgressIn<C> in = egress_load<C>(a, lane, gy, gx);
     uint8_t* q = a.out + (size_t)lane * a.out_lane_stride + (size_t)gy * a.out_step + (size_t)gx * C;
     float* f = a.fout ? a.fout + (((size_t)lane * a.h0 + gy) * a.w0 + gx) * C : nullptr;
-    egress_convert<C>(a, q, f, gx, in, up);
+    egress_convert(a, q, f, gx, in, up);
 }
 
-template <int C>
+// MC: motion channels (1 with C == 3: only the L planes of the band / cur planes are read, see egress_convert).
+template <int C, int MC>
 __global__ void __launch_bounds__(256) k_egress(const EgressArgs a) {
-    __shared__ __align__(16) float sC2[C][E2H][E2P];
-    __shared__ __align__(16) float sT[C][E2H][DP];    // horizontal pyrUp pass of the level-2 window rows
-    __shared__ __align__(16) float sD[C][DH][DP];
+    __shared__ __align__(16) float sC2[MC][E2H][E2P];
+    __shared__ __align__(16) float sT[MC][E2H][DP];    // horizontal pyrUp pass of the level-2 window rows
+    __shared__ __align__(16) float sD[MC][DH][DP];
     const int lane = blockIdx.z;
     const int x0 = blockIdx.x * TW, y0 = blockIdx.y * TH;
     const int w1 = a.l1.w, h1 = a.l1.h;
@@ -794,7 +797,7 @@ __global__ void __launch_bounds__(256) k_egress(const EgressArgs a) {
                     const int k = i / E2W, j = i - k * E2W;
                     const int o2 = upsrc(by2 + k, a.l2.h) * a.l2.pitch + upsrc(bx2 + j, a.l2.w);
 #pragma unroll
-                    for (int ch = 0; ch < C; ++ch) sC2[ch][k][j] = band_at(a.c2, base2 + (size_t)ch * a.l2.plane + o2);
+                    for (int ch = 0; ch < MC; ++ch) sC2[ch][k][j] = band_at(a.c2, base2 + (size_t)ch * a.l2.plane + o2);
                 }
                 __syncthreads();
             }
@@ -805,17 +808,17 @@ __global__ void __launch_bounds__(256) k_egress(const EgressArgs a) {
                 const bool odd = x1 & 1;
                 const int r = ky, cm = jx - 1, c0 = jx, cp = jx + 1;   // the window holds s[upsrc(i)]
 #pragma unroll
-                for (int ch = 0; ch < C; ++ch) {
+                for (int ch = 0; ch < MC; ++ch) {
                     const float sm = sC2[ch][r][cm], s0 = sC2[ch][r][c0], sp = sC2[ch][r][cp];
                     sT[ch][ky][j] = odd ? up2(s0, sp) : up3(sm, s0, sp);
                 }
             }
             __syncthreads();
         }
-        const float* __restrict__ ph[C];
-        const float* __restrict__ pl[C];
+        const float* __restrict__ ph[MC];
+        const float* __restrict__ pl[MC];
 #pragma unroll
-        for (int ch = 0; ch < C; ++ch) {
+        for (int ch = 0; ch < MC; ++ch) {
             ph[ch] = a.m1.a + (size_t)(lane * C + ch) * a.l1.plane;
             pl[ch] = a.m1.b ? a.m1.b + (size_t)(lane * C + ch) * a.l1.plane : nullptr;
         }
@@ -825,9 +828,9 @@ __global__ void __launch_bounds__(256) k_egress(const EgressArgs a) {
             const int k = i / DW, j = i - k * DW;
             const int y1 = upsrc(y0 / 2 - 1 + k, h1), x1 = upsrc(x0 / 2 - 1 + j, w1);
             const int o1 = y1 * a.l1.pitch + x1;
-            float v[C];
+            float v[MC];
 #pragma unroll
-            for (int ch = 0; ch < C; ++ch) {
+            for (int ch = 0; ch < MC; ++ch) {
                 v[ch] = __ldg(ph[ch] + o1);
                 if (from_state) v[ch] = band_of(v[ch], __ldg(pl[ch] + o1), g1);
             }
@@ -835,23 +838,23 @@ __global__ void __launch_bounds__(256) k_egress(const EgressArgs a) {
                 const int ky = (y1 >> 1) - by2;
                 const bool odd = y1 & 1;
 #pragma unroll
-                for (int ch = 0; ch < C; ++ch) {
+                for (int ch = 0; ch < MC; ++ch) {
                     const float r0 = sT[ch][ky - 1][j], r1 = sT[ch][ky][j], r2 = sT[ch][ky + 1][j];
                     v[ch] = __fmaf_rn(odd ? up2(r1, r2) : up3(r0, r1, r2), kInv64, v[ch]);
                 }
             }
 #pragma unroll
-            for (int ch = 0; ch < C; ++ch) sD[ch][k][j] = v[ch];
+            for (int ch = 0; ch < MC; ++ch) sD[ch][k][j] = v[ch];
         }
         __syncthreads();
     }
     const int tx = threadIdx.x & 15, ty = threadIdx.x >> 4;
     const int gx = x0 + 4 * tx;
     if (gx >= a.w0) return;
-    float up[C][2][4];
+    float up[MC][2][4];
     if (a.m1.a) {
 #pragma unroll
-        for (int ch = 0; ch < C; ++ch) {
+        for (int ch = 0; ch < MC; ++ch) {
             float e[3][4];
 #pragma unroll
             for (int q = 0; q < 3; ++q) {
@@ -873,9 +876,9 @@ __global__ void __launch_bounds__(256) k_egress(const EgressArgs a) {
     for (int ry = 0; ry < 2; ++ry) {
         const int gy = y0 + 2 * ty + ry;
         if (gy >= a.h0) continue;
-        float upr[C][4];
+        float upr[MC][4];
 #pragma unroll
-        for (int ch = 0; ch < C; ++ch)
+        for (int ch = 0; ch < MC; ++ch)
 #pragma unroll
             for (int i = 0; i < 4; ++i) upr[ch][i] = up[ch][ry][i];
         egress_pixels<C>(a, lane, gy, gx, upr);
@@ -925,7 +928,9 @@ constexpr int EG_ROWS = 64;   // output rows per warp (a multiple of 4)
 template <int C> struct StripM1 { float2 h[C], l[C]; };   // band-1 source of one cur_1 row at the lane's two columns
 template <int C> struct StripH2 { float v[C], vb[C], vr[C], vrb[C]; };   // one level-2 row at the lane's column (+ lane 31's right neighbour); b: lo state
 
-template <int C, int MINB>
+// MC: motion channels (1 with C == 3 when chroma is 0): the band / cur loads, both sliding windows and every pyrUp pass
+// run on the L planes only, and egress_convert passes A and B through.
+template <int C, int MC, int MINB>
 __global__ void __launch_bounds__(32, MINB) k_egress_strip(const EgressArgs a) {
     const unsigned full = 0xffffffffu;
     const int lane_id = threadIdx.x;
@@ -936,9 +941,9 @@ __global__ void __launch_bounds__(32, MINB) k_egress_strip(const EgressArgs a) {
     const int f_end = min(f0 + EG_ROWS, a.h0);
     const bool px_owner = lane_id >= 1 && lane_id <= 30 && gx < a.w0;
     if (!a.m1.a) {   // no motion (first frame, or fewer than two levels): conversion only
-        float zero[C][4];
+        float zero[MC][4];
 #pragma unroll
-        for (int ch = 0; ch < C; ++ch)
+        for (int ch = 0; ch < MC; ++ch)
 #pragma unroll
             for (int i = 0; i < 4; ++i) zero[ch][i] = 0.0f;
         if (px_owner)
@@ -954,9 +959,9 @@ __global__ void __launch_bounds__(32, MINB) k_egress_strip(const EgressArgs a) {
     const int x2l = x2 < 0 ? 0 : (x2 >= w2 ? w2 - 1 : x2);
     const int x2r = x2l + 1 >= w2 ? w2 - 1 : x2l + 1;                // lane 31's right neighbour column
     const int gxl = px_owner ? gx : 0;                               // input column for the (unused) loads of non-owners
-    size_t base1[C], base2[C];
+    size_t base1[MC], base2[MC];
 #pragma unroll
-    for (int ch = 0; ch < C; ++ch) {
+    for (int ch = 0; ch < MC; ++ch) {
         base1[ch] = (size_t)(lane * C + ch) * a.l1.plane + x1l;
         base2[ch] = (size_t)(lane * C + ch) * a.l2.plane;
     }
@@ -964,10 +969,10 @@ __global__ void __launch_bounds__(32, MINB) k_egress_strip(const EgressArgs a) {
     // ---- loads; the lines of the next iteration are requested into L1 while the current one is computed ----
     auto row1 = [&](int y1) { return (size_t)(y1 < h1 ? y1 : h1 - 1) * a.l1.pitch; };   // rows past the end are border copies
     auto ld_m1 = [&](int y1) {
-        StripM1<C> m;
+        StripM1<MC> m;
         const size_t ro = row1(y1);
 #pragma unroll
-        for (int ch = 0; ch < C; ++ch) {
+        for (int ch = 0; ch < MC; ++ch) {
             m.h[ch] = __ldg(reinterpret_cast<const float2*>(a.m1.a + base1[ch] + ro));
             m.l[ch] = from_state ? __ldg(reinterpret_cast<const float2*>(a.m1.b + base1[ch] + ro)) : make_float2(0.f, 0.f);
         }
@@ -976,16 +981,16 @@ __global__ void __launch_bounds__(32, MINB) k_egress_strip(const EgressArgs a) {
     auto pf_m1 = [&](int y1) {
         const size_t ro = row1(y1);
 #pragma unroll
-        for (int ch = 0; ch < C; ++ch) {
+        for (int ch = 0; ch < MC; ++ch) {
             prefetch_l1(a.m1.a + base1[ch] + ro);
             if (from_state) prefetch_l1(a.m1.b + base1[ch] + ro);
         }
     };
     auto ld_h2 = [&](int y2) {
-        StripH2<C> r;
+        StripH2<MC> r;
         const size_t ro = (size_t)upsrc(y2, h2) * a.l2.pitch;
 #pragma unroll
-        for (int ch = 0; ch < C; ++ch) {
+        for (int ch = 0; ch < MC; ++ch) {
             r.v[ch] = r.vb[ch] = r.vr[ch] = r.vrb[ch] = 0.f;
             if (has2) {
                 r.v[ch] = __ldg(a.c2.a + base2[ch] + ro + x2l);
@@ -1002,7 +1007,7 @@ __global__ void __launch_bounds__(32, MINB) k_egress_strip(const EgressArgs a) {
         const size_t ro = (size_t)upsrc(y2, h2) * a.l2.pitch;
         if (has2) {
 #pragma unroll
-            for (int ch = 0; ch < C; ++ch) {
+            for (int ch = 0; ch < MC; ++ch) {
                 prefetch_l1(a.c2.a + base2[ch] + ro + x2l);
                 if (st2) prefetch_l1(a.c2.b + base2[ch] + ro + x2l);
             }
@@ -1022,13 +1027,13 @@ __global__ void __launch_bounds__(32, MINB) k_egress_strip(const EgressArgs a) {
     // pixel stage and halve the number of resident warps of an issue-bound kernel.
     //   sH[i % 3]: horizontally expanded level-2 row i at the lane's two level-1 columns (even, odd)
     //   sE[j % 3]: horizontally expanded cur_1 row j at the lane's four output columns
-    __shared__ float2 sH[3][C][32];
-    __shared__ float4 sE[3][C][32];
+    __shared__ float2 sH[3][MC][32];
+    __shared__ float4 sE[3][MC][32];
     auto slot = [](int r) { return (r + 3) % 3; };      // rows >= -1
-    auto expand_h2 = [&](const StripH2<C>& in, int i) {
+    auto expand_h2 = [&](const StripH2<MC>& in, int i) {
         const int sl = slot(i);
 #pragma unroll
-        for (int ch = 0; ch < C; ++ch) {
+        for (int ch = 0; ch < MC; ++ch) {
             const float v = st2 ? band_of(in.v[ch], in.vb[ch], g2) : in.v[ch];
             float l = __shfl_up_sync(full, v, 1), r = __shfl_down_sync(full, v, 1);
             if (lane_id == 31) r = st2 ? band_of(in.vr[ch], in.vrb[ch], g2) : in.vr[ch];
@@ -1039,12 +1044,12 @@ __global__ void __launch_bounds__(32, MINB) k_egress_strip(const EgressArgs a) {
     };
     // cur_1 row y1 at the lane's two columns = pyrUp(cur_2) + m_1, then its horizontal expansion at the lane's four
     // output columns.  An even row 2i takes level-2 rows (i-1, i, i+1), an odd row 2i+1 rows (i, i+1).
-    auto cur1_row = [&](const StripM1<C>& m, int y1, float (&E)[C][4]) {
+    auto cur1_row = [&](const StripM1<MC>& m, int y1, float (&E)[MC][4]) {
         const bool odd = y1 & 1;
         const int i = y1 >> 1;
         const int sp = slot(odd ? i : i - 1), sq = slot(odd ? i + 1 : i), sr = slot(i + 1);
 #pragma unroll
-        for (int ch = 0; ch < C; ++ch) {
+        for (int ch = 0; ch < MC; ++ch) {
             float ca = m.h[ch].x, cb = m.h[ch].y;
             if (from_state) {
                 ca = band_of(ca, m.l[ch].x, g1);
@@ -1065,24 +1070,24 @@ __global__ void __launch_bounds__(32, MINB) k_egress_strip(const EgressArgs a) {
             E[ch][3] = up2(cb, right);
         }
     };
-    auto put_E = [&](int j, const float (&E)[C][4]) {
+    auto put_E = [&](int j, const float (&E)[MC][4]) {
         const int sl = slot(j);
 #pragma unroll
-        for (int ch = 0; ch < C; ++ch) sE[sl][ch][lane_id] = make_float4(E[ch][0], E[ch][1], E[ch][2], E[ch][3]);
+        for (int ch = 0; ch < MC; ++ch) sE[sl][ch][lane_id] = make_float4(E[ch][0], E[ch][1], E[ch][2], E[ch][3]);
     };
 
     const int j0 = f0 >> 1;                       // first level-1 row of the chunk (even)
     {
         const int ic = j0 >> 1;
-        const StripH2<C> ra = ld_h2(ic - 1), rb = ld_h2(ic), rc = ld_h2(ic + 1);
-        const StripM1<C> mp = ld_m1(j0 > 0 ? j0 - 1 : 1), m0 = ld_m1(j0);
+        const StripH2<MC> ra = ld_h2(ic - 1), rb = ld_h2(ic), rc = ld_h2(ic + 1);
+        const StripM1<MC> mp = ld_m1(j0 > 0 ? j0 - 1 : 1), m0 = ld_m1(j0);
         pf_m1(j0 + 1);
         pf_in(2 * j0);
         pf_in(min(2 * j0 + 1, a.h0 - 1));
         expand_h2(ra, ic - 1);
         expand_h2(rb, ic);
         expand_h2(rc, ic + 1);
-        float E[C][4];
+        float E[MC][4];
         // row j0-1 (odd, level-2 rows ic-1, ic); at the top of the image the slot of row -1 is filled with row 1 below
         if (j0 > 0) { cur1_row(mp, j0 - 1, E); put_E(j0 - 1, E); }
         cur1_row(m0, j0, E);
@@ -1092,14 +1097,16 @@ __global__ void __launch_bounds__(32, MINB) k_egress_strip(const EgressArgs a) {
     // Running row pointers (advanced once per iteration instead of rebuilt per access): band-1 source rows at the lane's
     // level-1 columns, the input rows at the lane's output columns, the output row.
     const size_t st1 = (size_t)a.l1.pitch, st16 = (size_t)a.pitch16;
-    const float* ph[C];
-    const float* pl[C];
+    const float* ph[MC];
+    const float* pl[MC];
     const int16_t* pin[C];
 #pragma unroll
     for (int ch = 0; ch < C; ++ch) {
-        const size_t ro = row1(j0 + 1);
-        ph[ch] = a.m1.a + base1[ch] + ro;
-        pl[ch] = from_state ? a.m1.b + base1[ch] + ro : ph[ch];
+        if (ch < MC) {
+            const size_t ro = row1(j0 + 1);
+            ph[ch] = a.m1.a + base1[ch] + ro;
+            pl[ch] = from_state ? a.m1.b + base1[ch] + ro : ph[ch];
+        }
         pin[ch] = C == 3 ? a.lab + (size_t)(lane * 3 + ch) * a.plane16 + (size_t)(2 * j0) * st16 + gxl : nullptr;
     }
     const uint8_t* pg = C == 1 ? a.in + (size_t)lane * a.in_lane_stride + (size_t)(2 * j0) * a.in_step : nullptr;   // gray input row
@@ -1109,13 +1116,13 @@ __global__ void __launch_bounds__(32, MINB) k_egress_strip(const EgressArgs a) {
         const int jn = j + 1;
         const bool two = 2 * j + 1 < f_end;                            // the chunk may end on an even row
         // what this iteration consumes (requested into L1 by the previous one) ...
-        StripM1<C> cm;
+        StripM1<MC> cm;
 #pragma unroll
-        for (int ch = 0; ch < C; ++ch) {
+        for (int ch = 0; ch < MC; ++ch) {
             cm.h[ch] = __ldg(reinterpret_cast<const float2*>(ph[ch]));
             cm.l[ch] = from_state ? __ldg(reinterpret_cast<const float2*>(pl[ch])) : make_float2(0.f, 0.f);
         }
-        StripH2<C> chh;
+        StripH2<MC> chh;
         if (!(jn & 1) && jn < h1) chh = ld_h2((jn >> 1) + 1);
         EgressIn<C> in0, in1;
         if (C == 3) {
@@ -1131,9 +1138,11 @@ __global__ void __launch_bounds__(32, MINB) k_egress_strip(const EgressArgs a) {
             if (jn & 1) pf_h2(((jn + 1) >> 1) + 1);
 #pragma unroll
             for (int ch = 0; ch < C; ++ch) {
-                if (adv1) { ph[ch] += st1; pl[ch] += st1; }
-                prefetch_l1(ph[ch]);
-                if (from_state) prefetch_l1(pl[ch]);
+                if (ch < MC) {
+                    if (adv1) { ph[ch] += st1; pl[ch] += st1; }
+                    prefetch_l1(ph[ch]);
+                    if (from_state) prefetch_l1(pl[ch]);
+                }
                 if (C == 3) {
                     pin[ch] += 2 * st16;
                     prefetch_l1(pin[ch]);
@@ -1143,10 +1152,10 @@ __global__ void __launch_bounds__(32, MINB) k_egress_strip(const EgressArgs a) {
             if (C == 1) { pg += 2 * a.in_step; prefetch_l1(pg + gxl); }
         }
         // row j+1 of cur_1 (or its border copy) -> Ep
-        float Ep[C][4];
+        float Ep[MC][4];
         if (jn >= h1) {
 #pragma unroll
-            for (int ch = 0; ch < C; ++ch) {
+            for (int ch = 0; ch < MC; ++ch) {
                 const float4 e = sE[s0][ch][lane_id];
                 Ep[ch][0] = e.x; Ep[ch][1] = e.y; Ep[ch][2] = e.z; Ep[ch][3] = e.w;
             }
@@ -1155,15 +1164,15 @@ __global__ void __launch_bounds__(32, MINB) k_egress_strip(const EgressArgs a) {
             cur1_row(cm, jn, Ep);
         }
 #pragma unroll
-        for (int ch = 0; ch < C; ++ch) sE[sp][ch][lane_id] = make_float4(Ep[ch][0], Ep[ch][1], Ep[ch][2], Ep[ch][3]);
+        for (int ch = 0; ch < MC; ++ch) sE[sp][ch][lane_id] = make_float4(Ep[ch][0], Ep[ch][1], Ep[ch][2], Ep[ch][3]);
         if (j == 0) {                                         // cur_1[-1] := cur_1[1]
 #pragma unroll
-            for (int ch = 0; ch < C; ++ch) sE[sm][ch][lane_id] = make_float4(Ep[ch][0], Ep[ch][1], Ep[ch][2], Ep[ch][3]);
+            for (int ch = 0; ch < MC; ++ch) sE[sm][ch][lane_id] = make_float4(Ep[ch][0], Ep[ch][1], Ep[ch][2], Ep[ch][3]);
         }
         if (px_owner) {
-            float up[C][4], t0[C][4];
+            float up[MC][4], t0[MC][4];
 #pragma unroll
-            for (int ch = 0; ch < C; ++ch) {
+            for (int ch = 0; ch < MC; ++ch) {
                 const float4 em = sE[sm][ch][lane_id], e0 = sE[s0][ch][lane_id];
                 t0[ch][0] = e0.x; t0[ch][1] = e0.y; t0[ch][2] = e0.z; t0[ch][3] = e0.w;
                 up[ch][0] = up3(em.x, e0.x, Ep[ch][0]);
@@ -1172,13 +1181,13 @@ __global__ void __launch_bounds__(32, MINB) k_egress_strip(const EgressArgs a) {
                 up[ch][3] = up3(em.w, e0.w, Ep[ch][3]);
             }
             float* f = a.fout ? a.fout + (((size_t)lane * a.h0 + 2 * j) * a.w0 + gx) * C : nullptr;
-            egress_convert<C>(a, pq, f, gx, in0, up);
+            egress_convert(a, pq, f, gx, in0, up);
             if (two) {
 #pragma unroll
-                for (int ch = 0; ch < C; ++ch)
+                for (int ch = 0; ch < MC; ++ch)
 #pragma unroll
                     for (int i = 0; i < 4; ++i) up[ch][i] = up2(t0[ch][i], Ep[ch][i]);
-                egress_convert<C>(a, pq + a.out_step, f ? f + (size_t)a.w0 * C : nullptr, gx, in1, up);
+                egress_convert(a, pq + a.out_step, f ? f + (size_t)a.w0 * C : nullptr, gx, in1, up);
             }
         }
         pq += 2 * a.out_step;
@@ -1291,15 +1300,15 @@ cudaError_t launch_down(const LevelArgs& a, cudaStream_t s) {
 }
 
 cudaError_t launch_collapse(const Level& lf, const Level& lc, const BandSrc& fine, const BandSrc& coarse, float* out, int planes,
-                            cudaStream_t s) {
-    dim3 grid(cdiv(lf.w, TW), cdiv(lf.h, TH), planes);
-    k_collapse<<<grid, 256, 0, s>>>(lf, lc, fine, coarse, out);
+                            cudaStream_t s, int plane_step) {
+    dim3 grid(cdiv(lf.w, TW), cdiv(lf.h, TH), planes / plane_step);
+    k_collapse<<<grid, 256, 0, s>>>(lf, lc, fine, coarse, out, plane_step);
     return cudaGetLastError();
 }
 
 cudaError_t launch_egress(const FrameIO& io, const DeviceTables& tb, const int16_t* lab, int pitch16, size_t plane16,
                           const BandSrc& m1, const Level& l1, const BandSrc& c2, const Level& l2, float chroma,
-                          float* fout, cudaStream_t s, int strip) {
+                          float* fout, cudaStream_t s, int strip, int motion_channels) {
     EgressArgs a;
     a.in = io.in; a.in_step = io.in_step; a.in_lane_stride = io.in_lane_stride;
     a.lab = lab; a.pitch16 = pitch16; a.plane16 = plane16;
@@ -1309,15 +1318,18 @@ cudaError_t launch_egress(const FrameIO& io, const DeviceTables& tb, const int16
     a.m1 = m1; a.l1 = l1; a.c2 = c2; a.l2 = l2; a.chroma = chroma; a.fout = fout;
     if (strip) {
         dim3 grid(cdiv(io.w, DS_COLS), cdiv(io.h, EG_ROWS), io.lanes);
-        // the register cap (resident warps per SM) is an A/B knob: 16 -> <= 128 registers, 20 -> 96, 24 -> 80
-        if (io.channels != 3) k_egress_strip<1, 24><<<grid, 32, 0, s>>>(a);
-        else if (strip == 16) k_egress_strip<3, 16><<<grid, 32, 0, s>>>(a);
-        else if (strip == 24) k_egress_strip<3, 24><<<grid, 32, 0, s>>>(a);
-        else k_egress_strip<3, 20><<<grid, 32, 0, s>>>(a);
+        // the register cap (resident warps per SM) of the three-channel kernel is an A/B knob: 16 -> <= 128 registers,
+        // 20 -> 96, 24 -> 80.  The L-only kernel (chroma 0) has one cap, 24, chosen on a B200 (DESIGN §4).
+        if (io.channels != 3) k_egress_strip<1, 1, 24><<<grid, 32, 0, s>>>(a);
+        else if (motion_channels == 1) k_egress_strip<3, 1, 24><<<grid, 32, 0, s>>>(a);
+        else if (strip == 16) k_egress_strip<3, 3, 16><<<grid, 32, 0, s>>>(a);
+        else if (strip == 24) k_egress_strip<3, 3, 24><<<grid, 32, 0, s>>>(a);
+        else k_egress_strip<3, 3, 20><<<grid, 32, 0, s>>>(a);
     } else {
         dim3 grid(cdiv(io.w, TW), cdiv(io.h, TH), io.lanes);
-        if (io.channels == 3) k_egress<3><<<grid, 256, 0, s>>>(a);
-        else k_egress<1><<<grid, 256, 0, s>>>(a);
+        if (io.channels != 3) k_egress<1, 1><<<grid, 256, 0, s>>>(a);
+        else if (motion_channels == 1) k_egress<3, 1><<<grid, 256, 0, s>>>(a);
+        else k_egress<3, 3><<<grid, 256, 0, s>>>(a);
     }
     return cudaGetLastError();
 }

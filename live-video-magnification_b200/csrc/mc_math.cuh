@@ -229,7 +229,11 @@ __device__ __forceinline__ float mc_ex2(float x) { float y; asm("ex2.approx.ftz.
 // NAN_AS_OPENCV: clip as OpenCV does (max(min(v, 1), 0): NaN -> 1.0, white).  Phase (Riesz) needs it — its L plane is
 // NaN wherever the blurred amplitude is 0, e.g. in letterbox bars — Motion (Laplace) cannot produce a NaN and keeps
 // the clip folded into the FFMA (.SAT, NaN -> 0) of its issue-bound egress kernel.
-template <bool NAN_AS_OPENCV = false>
+// G_R_FROM_Y: which product of the XYZ -> BGR dot products is rounded on its own (the other two are fused onto it, X
+// before Z, or Y before Z): X for all three rows, or X for b and Y for g and r.  The rounding is pinned with intrinsics
+// so that every instantiation of one kernel gives the same bits whatever code surrounds it (left to the compiler, the
+// choice followed the surrounding code); the Motion egress kernels use the second form, the Phase egress the first.
+template <bool NAN_AS_OPENCV = false, bool G_R_FROM_Y = false>
 __device__ __forceinline__ void lab_to_bgr_fast(float L, float a, float b, const LabInvCoeffs& k,
                                                 const float4* __restrict__ gtab, float& ob, float& og, float& orr) {
     const float y_lin = L * (1.0f / 903.3f);
@@ -243,9 +247,11 @@ __device__ __forceinline__ void lab_to_bgr_fast(float L, float a, float b, const
     const float fth = 6.0f / 29.0f;
     const float X = fx <= fth ? (fx - 16.0f / 116.0f) * (1.0f / 7.787f) : fx * fx * fx;
     const float Z = fz <= fth ? (fz - 16.0f / 116.0f) * (1.0f / 7.787f) : fz * fz * fz;
-    float vb = k.c[0] * X + k.c[1] * Y + k.c[2] * Z;
-    float vg = k.c[3] * X + k.c[4] * Y + k.c[5] * Z;
-    float vr = k.c[6] * X + k.c[7] * Y + k.c[8] * Z;
+    float vb = __fmaf_rn(k.c[2], Z, __fmaf_rn(k.c[1], Y, __fmul_rn(k.c[0], X)));
+    float vg = G_R_FROM_Y ? __fmaf_rn(k.c[5], Z, __fmaf_rn(k.c[3], X, __fmul_rn(k.c[4], Y)))
+                          : __fmaf_rn(k.c[5], Z, __fmaf_rn(k.c[4], Y, __fmul_rn(k.c[3], X)));
+    float vr = G_R_FROM_Y ? __fmaf_rn(k.c[8], Z, __fmaf_rn(k.c[6], X, __fmul_rn(k.c[7], Y)))
+                          : __fmaf_rn(k.c[8], Z, __fmaf_rn(k.c[7], Y, __fmul_rn(k.c[6], X)));
     if (NAN_AS_OPENCV) {
         // NOT fmaxf(fminf(v, 1), 0): ptxas folds that pair into the producing FFMA as .SAT, and .SAT turns NaN into 0
         // (black) where OpenCV's max(min(v,1),0) gives 1 (white).  The explicit NaN select survives the fold

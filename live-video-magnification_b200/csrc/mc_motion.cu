@@ -227,6 +227,10 @@ mc_status MotionMode::run_group(const ModeCtx& ctx, const FrameIO& io_all, const
         LAUNCH("copy", levels, launch_copy_planes(off(lo[(size_t)levels], levels), off(G[(size_t)levels], levels), n, ctx.stream));
     }
     if (ctx.analysis_only && !first) return MC_OK;
+    // chroma 0 multiplies the a and b planes of the motion image by 0 before input + motion (MagnifyCore.hpp:140-148),
+    // which leaves the input's a and b exactly as they are (DESIGN §4): the synthesis then runs on the L planes alone.
+    // The a and b state above keeps evolving, so a later frame with chroma != 0 is unaffected.  NaN compares unequal.
+    const int motion_channels = (channels == 3 && (float)p.chromAttenuation == 0.0f) ? 1 : channels;
     BandSrc m1, c2;
     if (!first && levels >= 2) {
         // synthesis: residual and finest band are zero (MagnifyCore.hpp:130-131), so the collapse starts from
@@ -236,14 +240,15 @@ mc_status MotionMode::run_group(const ModeCtx& ctx, const FrameIO& io_all, const
         };
         auto cur = [&](int l) { return l == levels - 1 ? band(l) : BandSrc{off(M[(size_t)l], l), nullptr, 1.0f}; };
         for (int l = levels - 2; l >= 2; --l)
-            LAUNCH("collapse", l, launch_collapse(lv[(size_t)l], lv[(size_t)l + 1], band(l), cur(l + 1), off(M[(size_t)l], l), planes, ctx.stream));
+            LAUNCH("collapse", l, launch_collapse(lv[(size_t)l], lv[(size_t)l + 1], band(l), cur(l + 1), off(M[(size_t)l], l), planes, ctx.stream,
+                                                  channels / motion_channels));
         m1 = band(1);
         if (levels >= 3) c2 = cur(2);
     }
     const Level& l1 = lv[levels >= 1 ? 1 : 0];
     const Level& l2 = lv[levels >= 2 ? 2 : 0];
     LAUNCH("egress", 0, launch_egress(io, *ctx.tables, lab, pitch16, plane16, m1, l1, c2, l2, (float)p.chromAttenuation, fout,
-                                      ctx.stream, ctx.egress_strip));
+                                      ctx.stream, ctx.egress_strip, motion_channels));
     return MC_OK;
 }
 
